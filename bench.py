@@ -20,7 +20,16 @@ cpu_baseline       : the reference's own CPU implementation (oracle/_ref/audiowm
 add / get          : the two halves of a step timed separately (north_star's target is on `get`)
 cli_e2e            : `bin/audiowmark add` + `cmp` as processes on a tmpfs WAV: process start, CUDA context creation, file I/O included
 
-python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--minutes M]
+python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--minutes M] [--dump-outputs DIR]
+
+--dump-outputs DIR : after the timed steps, what the last timed resident step returned, as DIR/<name>.npy (float32 / float64,
+                     about 16 MB in all; the input is a pure function of the arguments, so two builds compare output for output):
+  marked_frame, marked_audio      a fixed, seeded sample of 2^20 frame numbers of the marked audio `add` wrote and their samples
+                                  (frames x channels; with several GPUs, of rank 0's range)
+  match_pos_s, match_quality, match_error, match_rating, match_speed
+                                  the fields of the matches of the `get --json` document, in its order (pos in seconds)
+  match_type                      index of the type string in MATCH_TYPES
+  match_bits                      the decoded payload, one 0 / 1 entry per bit (matches x 128)
 """
 import argparse
 import json
@@ -95,11 +104,8 @@ def run_reference(steps, warmup, minutes):
     """The reference's own CPU `add` + `get` (unmodified sources in oracle/_ref) on a bounded sample."""
     import numpy as np
     import awm_oracle as O
-    if not os.path.exists(REF_BIN):
-        import build_oracle
-        build_oracle.build_reference()
-    if not os.path.exists(REF_BIN):
-        raise RuntimeError("oracle/_ref/audiowmark is missing (built by __graft_entry__.build() where /root/reference is mounted)")
+    if not os.path.exists(REF_BIN):           # built by __graft_entry__.build(); the benchmark itself writes nothing into the tree
+        raise RuntimeError("oracle/_ref/audiowmark is missing (__graft_entry__.build() makes it where the reference sources are available)")
     seconds = minutes * 60.0
     n = int(seconds * RATE)
     tmp = tempfile.mkdtemp(prefix="awm_ref_", dir="/dev/shm" if os.path.isdir("/dev/shm") else None)
@@ -223,6 +229,28 @@ def bind_to_gpu_numa_node(gpu_index):
         return "cpu affinity set to the GPU's local CPUs (%d)" % len(os.sched_getaffinity(0))
     except Exception as e:
         return "not bound: %s" % e
+
+
+DUMP_FRAMES = 1 << 20                     # 8 MB of stereo float32 + 8 MB of frame numbers (the marked hour is 1.27 GB)
+MATCH_TYPES = [c + b + s for c in ("", "CLIP-") for b in ("A", "B", "AB", "ALL") for s in ("", "-SPEED")]
+
+
+def step_outputs(y_dev, n_frames, doc):
+    """What a caller of the timed step receives, as arrays (see --dump-outputs): a seeded sample of the marked audio and the
+    matches of the `get --json` document `doc` (None: no document on this rank)."""
+    import numpy as np
+    import torch
+    idx = np.sort(np.random.default_rng(2024).choice(n_frames, min(n_frames, DUMP_FRAMES), replace=False))
+    out = {"marked_frame": idx.astype(np.float64),
+           "marked_audio": y_dev.index_select(0, torch.from_numpy(idx).to(y_dev.device)).cpu().numpy()}
+    matches = json.loads(doc)["matches"] if doc is not None else []
+    out["match_pos_s"] = np.array([sum(int(v) * 60 ** i for i, v in enumerate(reversed(m["pos"].split(":")))) for m in matches], np.float64)
+    for f in ("quality", "error", "rating", "speed"):
+        out["match_" + f] = np.array([m[f] for m in matches], np.float64)
+    out["match_type"] = np.array([MATCH_TYPES.index(m["type"]) for m in matches], np.float64)
+    out["match_bits"] = np.array([[(int(c, 16) >> (3 - b)) & 1 for c in m["bits"] for b in range(4)] for m in matches],
+                                 np.float32).reshape(len(matches), 4 * len(PAYLOAD))
+    return out
 
 
 def main_gpu(args):
@@ -370,6 +398,7 @@ def main_gpu(args):
     for _ in range(args.warmup):
         step_resident()
     ms, wall, doc, launches, prof = timed(step_resident, args.steps, True)
+    dumped = step_outputs(y_dev, n_loc, doc) if args.dump_outputs and rank == 0 else None
     ok, n_real = check(doc)
     if args.resident_only:
         ms_e2e = ms_e2e16 = float("nan")
@@ -573,6 +602,10 @@ def main_gpu(args):
         "cpu_baseline": cpu,
         "clocks": clk,
     }
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -587,6 +620,7 @@ def main():
     ap.add_argument("--minutes", type=float, default=0.0, help="audio length per GPU (default 60 = BASELINE configs[1], both arms)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--resident-only", action="store_true", help="only the resident legs (for the ncu launch list: every launch it sees belongs to a warm-up or timed resident step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     if args.impl == "reference":
         main_reference(args)
