@@ -179,18 +179,19 @@ k_stft_mags_tc (const float *__restrict__ pcm, long long n_frames, int C, int n_
                       im[j] = __fmul_rn (v.y, wn);
                     }
                   __syncwarp();                                   // all lanes hold their samples before the transposes reuse the buffer
+                  const unsigned zero = pair_zero_mask (re, im);
                   fft1024_warp (re, im, s.tw, s.xbuf, lane, [&] { if (nxt_tma) prefetch (nxt); });
                   // dB with MUFU.LG2 (__log2f): its error (~2e-7 relative) is two orders below the 2^-16 absolute resolution the
                   // value is about to be stored with (fp16 hi + lo), and saves ~170 of the ~2000 instructions of a frame
                   auto db = [] (float re_, float im_) { const float a2 = __fmaf_rn (re_, re_, __fmul_rn (im_, im_)); return a2 > 0.0f ? __log2f (a2) * 3.01029995663981f : -96.f; };
                   float ar, ai, br, bi;
-                  unpack_pair<0> (re, im, lane, ar, ai, br, bi);
+                  unpack_pair<0> (re, im, lane, ar, ai, br, bi, zero);
                   acc[0] = db (ar, ai) + db (br, bi);
-                  unpack_pair<1> (re, im, lane, ar, ai, br, bi);
+                  unpack_pair<1> (re, im, lane, ar, ai, br, bi, zero);
                   acc[1] = db (ar, ai) + db (br, bi);
-                  unpack_pair<2> (re, im, lane, ar, ai, br, bi);
+                  unpack_pair<2> (re, im, lane, ar, ai, br, bi, zero);
                   acc[2] = db (ar, ai) + db (br, bi);
-                  unpack_pair<3> (re, im, lane, ar, ai, br, bi);
+                  unpack_pair<3> (re, im, lane, ar, ai, br, bi, zero);
                   acc[3] = db (ar, ai) + db (br, bi);
                 }
               else

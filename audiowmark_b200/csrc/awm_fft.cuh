@@ -131,11 +131,29 @@ fft1024_warp (float (&re)[32], float (&im)[32], const float2 *tw, float *xbuf, i
   fft1024_warp (re, im, tw, xbuf, lane, [] {});
 }
 
+// Which of the two real inputs packed into (re, im) -- before the transform -- are zero in every sample of the warp: bit 0 the real
+// part a, bit 1 the imaginary part b.  ORing the bit patterns and dropping the sign bit counts -0.0 as zero.
+__device__ __forceinline__ unsigned
+pair_zero_mask (const float (&re)[32], const float (&im)[32])
+{
+  unsigned oa = 0, ob = 0;
+#pragma unroll
+  for (int j = 0; j < 32; j++)
+    {
+      oa |= __float_as_uint (re[j]);
+      ob |= __float_as_uint (im[j]);
+    }
+  return (__all_sync (0xffffffffu, (oa << 1) == 0) ? 1u : 0u) | (__all_sync (0xffffffffu, (ob << 1) == 0) ? 2u : 0u);
+}
+
 // Split the packed spectrum Z = FFT (a + i b) into the spectra of the two real inputs for
 // bin k = lane + 32*K2:   A[k] = (Z[k] + conj Z[N-k]) / 2,   B[k] = (Z[k] - conj Z[N-k]) / (2i)
 // Z[N-k] lives in lane (32-lane)&31 (register for k2' = 31-K2; lane 0 keeps k2' = (32-K2)&31).
+// `zero` (pair_zero_mask of the input): an input that is zero in every sample has an exactly zero spectrum -- the reference then
+// gets -96 dB in every bin (db_from_complex) -- while the formula above would return the rounding error of the other input's
+// transform (the float FFT of a real input is not exactly Hermitian) at float rounding level of that input's magnitude.
 template<int K2> __device__ __forceinline__ void
-unpack_pair (const float (&re)[32], const float (&im)[32], int lane, float& ar, float& ai, float& br, float& bi)
+unpack_pair (const float (&re)[32], const float (&im)[32], int lane, float& ar, float& ai, float& br, float& bi, unsigned zero = 0)
 {
   constexpr int I = brev5 (K2 & 31), IP = brev5 ((31 - K2) & 31), IP0 = brev5 ((32 - K2) & 31);
   const float sr = (lane == 0) ? re[IP0] : re[IP];
@@ -148,6 +166,10 @@ unpack_pair (const float (&re)[32], const float (&im)[32], int lane, float& ar, 
   ai = 0.5f * (zi - pi);
   br = 0.5f * (zi + pi);
   bi = -0.5f * (zr - pr);
+  if (zero & 1u)
+    ar = ai = 0.f;
+  if (zero & 2u)
+    br = bi = 0.f;
 }
 
 // db_from_complex (reference src/wmcommon.hh:204-224)

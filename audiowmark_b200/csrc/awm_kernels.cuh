@@ -110,18 +110,19 @@ frame_db_sum (const float *__restrict__ pcm, long long n_frames, int C, long lon
       const int chB = (chA + 1 < C) ? chA + 1 : -1;
       float re[32], im[32];
       load_pair (pcm, n_frames, C, start, chA, chB, s.win, re, im, lane);
+      const unsigned zero = pair_zero_mask (re, im);
       fft1024_warp (re, im, s.tw, s.xbuf, lane);
       float ar, ai, br, bi;
-      unpack_pair<0> (re, im, lane, ar, ai, br, bi);
+      unpack_pair<0> (re, im, lane, ar, ai, br, bi, zero);
       acc[0] += db_from_complex (ar, ai, -96.f);
       if (chB >= 0) acc[0] += db_from_complex (br, bi, -96.f);
-      unpack_pair<1> (re, im, lane, ar, ai, br, bi);
+      unpack_pair<1> (re, im, lane, ar, ai, br, bi, zero);
       acc[1] += db_from_complex (ar, ai, -96.f);
       if (chB >= 0) acc[1] += db_from_complex (br, bi, -96.f);
-      unpack_pair<2> (re, im, lane, ar, ai, br, bi);
+      unpack_pair<2> (re, im, lane, ar, ai, br, bi, zero);
       acc[2] += db_from_complex (ar, ai, -96.f);
       if (chB >= 0) acc[2] += db_from_complex (br, bi, -96.f);
-      unpack_pair<3> (re, im, lane, ar, ai, br, bi);
+      unpack_pair<3> (re, im, lane, ar, ai, br, bi, zero);
       acc[3] += db_from_complex (ar, ai, -96.f);
       if (chB >= 0) acc[3] += db_from_complex (br, bi, -96.f);
     }
@@ -163,6 +164,7 @@ k_fft_r2c (const float *__restrict__ in, float *__restrict__ out, long long coun
       re[j] = a[32 * j + lane];
       im[j] = have_b ? b[32 * j + lane] : 0.f;
     }
+  const unsigned zero = pair_zero_mask (re, im);
   fft1024_warp (re, im, s.tw, s.xbuf, lane);
   float2 *oa = reinterpret_cast<float2 *> (out + 2 * p * (kFrame + 2)), *ob = oa + (kFrame / 2 + 1);
   auto emit = [&] (int k, bool pred, float ar, float ai, float br, float bi)
@@ -175,11 +177,11 @@ k_fft_r2c (const float *__restrict__ in, float *__restrict__ out, long long coun
         }
     };
   float ar, ai, br, bi;
-#define AWM_EMIT(K2) unpack_pair<K2> (re, im, lane, ar, ai, br, bi); emit (lane + 32 * K2, true, ar, ai, br, bi);
+#define AWM_EMIT(K2) unpack_pair<K2> (re, im, lane, ar, ai, br, bi, zero); emit (lane + 32 * K2, true, ar, ai, br, bi);
   AWM_EMIT (0) AWM_EMIT (1) AWM_EMIT (2) AWM_EMIT (3) AWM_EMIT (4) AWM_EMIT (5) AWM_EMIT (6) AWM_EMIT (7)
   AWM_EMIT (8) AWM_EMIT (9) AWM_EMIT (10) AWM_EMIT (11) AWM_EMIT (12) AWM_EMIT (13) AWM_EMIT (14) AWM_EMIT (15)
 #undef AWM_EMIT
-  unpack_pair<16> (re, im, lane, ar, ai, br, bi);
+  unpack_pair<16> (re, im, lane, ar, ai, br, bi, zero);
   emit (512, lane == 0, ar, ai, br, bi);
 }
 
@@ -572,12 +574,13 @@ k_decode_fft (const float *__restrict__ pcm, long long n_frames, int C, const lo
   const long long start = blk_start[b] + (long long) f * kFrame;
   float re[32], im[32];
   load_pair (pcm, n_frames, C, start, chA, chB, s.win, re, im, lane);
+  const unsigned zero = pair_zero_mask (re, im);
   fft1024_warp (re, im, s.tw, s.xbuf, lane);
   float *da = D + (((size_t) b * frames_per_block + f) * C + chA) * kBands;
   float *dbb = da + kBands;
   float ar, ai, br, bi;
 #define AWM_DB(K2) \
-  unpack_pair<K2> (re, im, lane, ar, ai, br, bi); \
+  unpack_pair<K2> (re, im, lane, ar, ai, br, bi, zero); \
   { const int band = lane + 32 * K2 - kMinBand; \
     if (band >= 0 && band < kBands) { da[band] = db_from_complex (ar, ai, -96.f); if (chB >= 0) dbb[band] = db_from_complex (br, bi, -96.f); } }
   AWM_DB (0) AWM_DB (1) AWM_DB (2) AWM_DB (3)

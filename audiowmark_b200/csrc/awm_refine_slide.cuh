@@ -73,13 +73,14 @@ k_refine_slide (const float *__restrict__ pcm, long long n_frames,
             im[j] = 0.f;
           }
       }
+    const unsigned zero = pair_zero_mask (re, im);      // a channel that is zero over the frame slides on from an exactly zero spectrum
     fft1024_warp (re, im, s.tw, s.xbuf, lane);
     float4 *sc = reinterpret_cast<float4 *> (s.xbuf);           // the transpose buffer is free again: [128] (Lre, Lim, Rre, Rim)
     float ar, ai, br, bi;
-    unpack_pair<0> (re, im, lane, ar, ai, br, bi); sc[lane]      = make_float4 (ar, ai, br, bi);
-    unpack_pair<1> (re, im, lane, ar, ai, br, bi); sc[lane + 32] = make_float4 (ar, ai, br, bi);
-    unpack_pair<2> (re, im, lane, ar, ai, br, bi); sc[lane + 64] = make_float4 (ar, ai, br, bi);
-    unpack_pair<3> (re, im, lane, ar, ai, br, bi); sc[lane + 96] = make_float4 (ar, ai, br, bi);
+    unpack_pair<0> (re, im, lane, ar, ai, br, bi, zero); sc[lane]      = make_float4 (ar, ai, br, bi);
+    unpack_pair<1> (re, im, lane, ar, ai, br, bi, zero); sc[lane + 32] = make_float4 (ar, ai, br, bi);
+    unpack_pair<2> (re, im, lane, ar, ai, br, bi, zero); sc[lane + 64] = make_float4 (ar, ai, br, bi);
+    unpack_pair<3> (re, im, lane, ar, ai, br, bi, zero); sc[lane + 96] = make_float4 (ar, ai, br, bi);
     __syncwarp();
 #pragma unroll
     for (int b = 0; b < kSlideBins; b++)

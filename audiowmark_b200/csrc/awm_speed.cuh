@@ -215,11 +215,11 @@ split_rows_db (float are, float aim, float bre, float bim, float& db_even, float
 // is needed, so the twiddle drops out.  Bins 20..100 live in registers k2 = 0..3 (k = lane + 32 k2), their partners
 // k + 512 in k2 + 16.
 template<int K2> __device__ __forceinline__ void
-speed_db_k2 (const float (&re)[32], const float (&im)[32], int lane, bool second_channel, float& acc_even, float& acc_odd)
+speed_db_k2 (const float (&re)[32], const float (&im)[32], int lane, bool second_channel, unsigned zero, float& acc_even, float& acc_odd)
 {
   float a0r, a0i, b0r, b0i, a1r, a1i, b1r, b1i;
-  unpack_pair<K2> (re, im, lane, a0r, a0i, b0r, b0i);
-  unpack_pair<K2 + 16> (re, im, lane, a1r, a1i, b1r, b1i);
+  unpack_pair<K2> (re, im, lane, a0r, a0i, b0r, b0i, zero);
+  unpack_pair<K2 + 16> (re, im, lane, a1r, a1i, b1r, b1i, zero);
   float e, o;
   split_rows_db (a0r, a0i, a1r, a1i, e, o);
   acc_even = __fadd_rn (acc_even, e);
@@ -272,11 +272,12 @@ k_speed_mags (const MagJob *__restrict__ jobs, int C, const awm_sync_entry *__re
             re[j] = xr;
             im[j] = xi;
           }
+        const unsigned zero = pair_zero_mask (re, im);
         fft1024_warp (re, im, g_tw, xbuf, lane);
-        speed_db_k2<0> (re, im, lane, two, acc_e[0], acc_o[0]);
-        speed_db_k2<1> (re, im, lane, two, acc_e[1], acc_o[1]);
-        speed_db_k2<2> (re, im, lane, two, acc_e[2], acc_o[2]);
-        speed_db_k2<3> (re, im, lane, two, acc_e[3], acc_o[3]);
+        speed_db_k2<0> (re, im, lane, two, zero, acc_e[0], acc_o[0]);
+        speed_db_k2<1> (re, im, lane, two, zero, acc_e[1], acc_o[1]);
+        speed_db_k2<2> (re, im, lane, two, zero, acc_e[2], acc_o[2]);
+        speed_db_k2<3> (re, im, lane, two, zero, acc_e[3], acc_o[3]);
       }
 #pragma unroll
     for (int k2 = 0; k2 < 4; k2++)

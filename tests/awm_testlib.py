@@ -51,6 +51,111 @@ def noise(seconds, channels=2, seed=1234, amp=0.5):
     return ((rng.random((n, channels), dtype=np.float32) - 0.5) * (2 * amp)).astype(np.float32)
 
 
+# --------------------------------------------------------------------------- deterministic "music-like" signals
+# Seeded numpy in float64, returned on the 16 bit grid (float32, as a 16 bit file reads back); where results for them are stored,
+# so is the SHA-256 of the int16 samples, so a box whose numpy / scipy computes a different signal fails loudly.
+# Tones are periodic in samples: their phase is looked up from the integer sample index, never computed as sin of a large argument.
+
+RATE = 44100
+
+# (cycles, period): a tone with `cycles` periods every `period` samples; bin k of the 1024 point analysis is k * 44100 / 1024 Hz,
+# the sync / data bands are bins 20..100
+MUSIC_TONES = ((40, 1024), (71, 1024),        # on the bin centres k = 40, 71
+               (105, 2048), (177, 2048),      # half-way between bins: k = 52.5, 88.5
+               (11, 2205),                    # 220 Hz, below the band
+               (20, 147))                     # 6 kHz, above it
+TONE_475 = (95, 2048)                         # k = 47.5: half-way between two in-band bins
+
+
+def db(v):
+    return 10.0 ** (v / 20.0)
+
+
+def periodic_tone(n, cycles, period, phase_num=0, channels=1):
+    """sin(2 pi (t * cycles / period + phase)) for t = 0..n-1, phase = (phase_num + channel) / 7 of a cycle -> float64 [n, channels]"""
+    t = np.arange(n, dtype=np.int64)
+    table = np.sin(2 * np.pi * np.arange(period, dtype=np.float64) / period)
+    out = np.empty((n, channels))
+    for c in range(channels):
+        off = (period * (phase_num + c)) // 7
+        out[:, c] = table[(t * cycles + off) % period]
+    return out
+
+
+def pink(n, channels, rng):
+    """independent 1/f noise per channel: seeded white noise through a fixed 3-pole / 3-zero IIR with a roughly
+    -3 dB/octave response, normalised to RMS 1"""
+    from scipy.signal import lfilter
+    b = [0.049922035, -0.095993537, 0.050612699, -0.004408786]
+    a = [1.0, -2.494956002, 2.017265875, -0.522189400]
+    w = rng.standard_normal((n + 4096, channels))
+    p = lfilter(b, a, w, axis=0)[4096:]              # the filter's start-up transient is cut off
+    return p / np.sqrt(np.mean(p * p, axis=0))
+
+
+def to16(x):
+    """float64 -> the 16 bit grid (clipped like a 16 bit file write) -> float32"""
+    return O.int16_to_float(O.quantize_sndfile16(np.asarray(x, np.float64).astype(np.float32)))
+
+
+def music_f64(seconds, channels=2, seed=1):
+    """pink noise at -20 dBFS RMS per channel plus six steady -12 dBFS tones shared by all channels (per-channel phases);
+    the sum is scaled to a -1 dBFS peak, so the tones end up near -16 dBFS"""
+    n = int(seconds * RATE)
+    rng = np.random.default_rng(seed)
+    x = db(-20) * pink(n, channels, rng)
+    for j, (cycles, period) in enumerate(MUSIC_TONES):
+        x += db(-12) * periodic_tone(n, cycles, period, phase_num=j, channels=channels)
+    return x * (db(-1) / np.abs(x).max())
+
+
+def music(seconds, channels=2, seed=1):
+    return to16(music_f64(seconds, channels, seed))
+
+
+def tone(seconds, channels=2, seed=2):
+    """one -6 dBFS tone half-way between two in-band bins over a noise floor of 1 LSB RMS: the widest in-band dynamic range a
+    16 bit file holds, and the input on which the sliding DFT's cancellation errors are largest"""
+    n = int(seconds * RATE)
+    rng = np.random.default_rng(seed)
+    x = db(-6) * periodic_tone(n, *TONE_475, channels=channels) + rng.standard_normal((n, channels)) / 32768
+    return to16(x)
+
+
+def quiet(seconds, channels=2, seed=3):
+    """music at a -60 dBFS peak: a few dozen LSB"""
+    x = music_f64(seconds, channels, seed)
+    return to16(x * (db(-60) / np.abs(x).max()))
+
+
+def dc_clip(seconds, channels=2, seed=4):
+    """music + 0.3 DC, amplified until 1 % of the samples exceed full scale, hard clipped"""
+    x = music_f64(seconds, channels, seed)
+    lo, hi = 0.5, 8.0                                  # bisect the gain: fraction of |g x + 0.3| > 1 is monotonic in g
+    for _ in range(60):
+        g = 0.5 * (lo + hi)
+        if np.mean(np.abs(g * x + 0.3) > 1.0) < 0.01:
+            lo = g
+        else:
+            hi = g
+    return to16(np.clip(lo * x + 0.3, -1.0, 1.0))
+
+
+def one_sided(seconds, kind, seed=5):
+    """stereo from one music channel L: kind "zero" (R = 0), "m50" (R = L at -50 dB: tens of LSB), "same" (R = L), "neg" (R = -L)"""
+    L = music_f64(seconds, 1, seed)[:, 0]
+    R = {"zero": 0.0 * L, "m50": db(-50) * L, "same": L, "neg": -L}[kind]
+    return to16(np.stack([L, R], axis=1))
+
+
+SIGNALS = {"music": music, "tone": tone, "quiet": quiet, "dc_clip": dc_clip, "one_sided": one_sided}
+
+
+def signal(spec):
+    """spec = {"fn": name in SIGNALS, "args": keyword arguments} (how tests/golden/golden_large.json names its inputs)"""
+    return SIGNALS[spec["fn"]](**spec["args"])
+
+
 def rms(x):
     x = np.asarray(x, np.float64)
     return float(np.sqrt(np.mean(x * x))) if x.size else 0.0

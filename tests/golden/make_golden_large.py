@@ -1,9 +1,14 @@
-"""Generate tests/golden/golden_large.json: BASELINE.json's configs 2-4 at their stated sizes, the digital-silence cases and the
-exact sync positions, all from the UNMODIFIED reference sources built by oracle/Makefile.ref
+"""Generate tests/golden/golden_large.json: BASELINE.json's configs 2-4 at their stated sizes, the digital-silence cases, the
+music-like / tonal / quiet / clipped / one-sided stereo / mono / 3-channel cases (MUSIC_CASES) and the exact sync positions, all
+from the UNMODIFIED reference sources built by oracle/Makefile.ref
   oracle/_ref/audiowmark   the reference CLI
   oracle/_ref/sync_dump    the reference's SyncFinder::search behind a print loop (oracle/ref_shims/sync_dump.cc)
 
 Run here (needs /root/reference to build the binaries; about 10 minutes):   python tests/golden/make_golden_large.py
+Only some of MUSIC_CASES (about 10 s each, music600 2 minutes), the rest of the file kept:   python tests/golden/make_golden_large.py music130 ...
+A full run reproduces the MUSIC_CASES entries byte for byte; of the older entries, the hour's add_stderr holds the temporary
+directory of the run that made it, and the reference prints the rating of some of the hour's and speed600's patterns with a
+last digit that can change from run to run (143.98074 / 143.98073).
 Only hashes, JSON documents and score lists are stored; the tests regenerate the inputs from seeds with the oracle
 (bit exact against these hashes) on whatever box they run.
 """
@@ -27,6 +32,28 @@ REF = build_oracle.build_reference()
 DUMP = build_oracle.REF_SYNC_DUMP
 assert REF and os.path.exists(REF) and os.path.exists(DUMP), "reference binaries not available"
 PAYLOAD = "f0f0f0f0f0f0f0f0f0f0f0f0f0f0f0f0"
+PAYLOAD2 = "0123456789abcdef0123456789abcdef"
+TWO_KEYS = {"alpha": "000102030405060708090a0b0c0d0e0f", "beta": "101112131415161718191a1b1c1d1e1f"}
+
+
+def _sig(fn, **args):
+    return {"fn": fn, "args": args}
+
+
+# name -> input (tests/awm_testlib.py signal spec); every case is watermarked by the reference with PAYLOAD and read back
+MUSIC_CASES = {
+    "music130": _sig("music", seconds=130, channels=2, seed=1),
+    "tone170": _sig("tone", seconds=170, channels=2, seed=2),
+    "quiet130": _sig("quiet", seconds=130, channels=2, seed=3),
+    "dc_clip130": _sig("dc_clip", seconds=130, channels=2, seed=4),
+    "r_zero130": _sig("one_sided", seconds=130, kind="zero", seed=5),
+    "r_m50_130": _sig("one_sided", seconds=130, kind="m50", seed=5),
+    "r_same130": _sig("one_sided", seconds=130, kind="same", seed=5),
+    "r_neg130": _sig("one_sided", seconds=130, kind="neg", seed=5),
+    "mono170": _sig("music", seconds=170, channels=1, seed=6),
+    "ch3_170": _sig("music", seconds=170, channels=3, seed=7),
+    "music600": _sig("music", seconds=600, channels=2, seed=8),
+}
 
 
 def run(exe, *args, ok_codes=(0,)):
@@ -64,7 +91,43 @@ def get_case(tmp, wav, extra=()):
     return {"get_stdout": g.stdout, "json": json.load(open(js)), "get_args": list(extra)}
 
 
+def music_cases(G, tmp, names):
+    """MUSIC_CASES (and music600_two_keys with music600).  130 s: one full A block, and short enough (< 3.1 blocks) that the clip
+    decoder's two CLIP searches run too; 170 s: BLOCK search only, three sync blocks.  The temporary directory is cut out of the
+    stored add output, so that a second run stores the same bytes."""
+    p = lambda name: os.path.join(tmp, name)
+    for name in names:
+        spec = MUSIC_CASES[name]
+        x = T.signal(spec)
+        O.write_wav16(p("m.wav"), x)
+        a = run(REF, "add", p("m.wav"), p("mwm.wav"), PAYLOAD)
+        G[name] = dict(get_case(tmp, p("mwm.wav")), signal=spec, input_sha256=sha(O.quantize_sndfile16(x)), add_stderr=a.stderr.replace(tmp + "/", ""),
+                       output_sha256=sha(pcm16(p("mwm.wav"))), payload=PAYLOAD, sync=sync_dump(p("mwm.wav")))
+        if name == "music600":
+            # the same input watermarked twice with two named keys from key files (as two_keys30 in golden.json); get with both
+            k1, k2 = p("k1.key"), p("k2.key")
+            open(k1, "w").write('key %s\nname "alpha"\n' % TWO_KEYS["alpha"])
+            open(k2, "w").write('key %s\nname "beta"\n' % TWO_KEYS["beta"])
+            run(REF, "add", "--key", k1, p("m.wav"), p("k1wm.wav"), PAYLOAD)
+            a2 = run(REF, "add", "--key", k2, p("k1wm.wav"), p("k2wm.wav"), PAYLOAD2)
+            js = p("out.json")
+            g2 = run(REF, "get", "--key", k1, "--key", k2, "--json", js, p("k2wm.wav"))
+            G["music600_two_keys"] = {"signal": spec, "keys": TWO_KEYS, "payload": PAYLOAD, "payload2": PAYLOAD2,
+                                      "add_stderr": a2.stderr.replace(tmp + "/", ""), "output_sha256": sha(pcm16(p("k2wm.wav"))),
+                                      "get_stdout": g2.stdout, "json": json.load(open(js))}
+
+
 def main():
+    out = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden_large.json")
+    names = sys.argv[1:]
+    assert all(n in MUSIC_CASES for n in names), "unknown case; one of %s" % ", ".join(MUSIC_CASES)
+    if names:                                       # only these cases, the rest of the file stays as it is
+        G = json.load(open(out))
+        with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as tmp:
+            music_cases(G, tmp, names)
+        json.dump(G, open(out, "w"), indent=1, sort_keys=True)
+        print("wrote", out, os.path.getsize(out), "bytes")
+        return
     G = {"reference": "swesterfeld/audiowmark 0.6.5 sources compiled unmodified by oracle/Makefile.ref (FFT: oracle/ref_shims/fftw_shim.cc, "
                       "resampler: oracle/ref_shims/awm_vresampler.hh); sync positions from oracle/ref_shims/sync_dump.cc"}
     with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as tmp:
@@ -120,7 +183,7 @@ def main():
             case = get_case(tmp, p("sp.wav"), extra=("--detect-speed",))
             case.update(speed=speed, input_sha256=sha(s16), n_frames=int(len(s16)))
             G["speed600"]["cases"].append(case)
-    out = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden_large.json")
+        music_cases(G, tmp, MUSIC_CASES)
     json.dump(G, open(out, "w"), indent=1, sort_keys=True)
     print("wrote", out, os.path.getsize(out), "bytes")
 

@@ -6,6 +6,9 @@ oracle/_ref/audiowmark and oracle/_ref/sync_dump):
   config 3   30 s clip cut from the 1 h output by test-clip (seed 0): clip decoder, 8 sync scores
   config 4   --detect-speed on 10 min stereo at speeds 0.9 / 0.9764 / 1.01 / 1.1 (the edges of the +-10 % scan range included)
   silence    170 s of zeros; 60 s of watermarked noise followed by 60 s of zeros
+  music      music-like (pink noise + steady tones), a -6 dBFS tone over a 1 LSB floor, -60 dBFS music, clipped music with DC,
+             one-sided stereo (R silent, R at -50 dB, R = L, R = -L), mono and 3 channels: 130 s (clip decoder runs too) or 170 s
+             (three sync blocks); 10 min stereo music, also watermarked with two named keys
 
 The inputs are regenerated here from seeds with the oracle (keyed noise generator, bit exact embedder, resampler) and checked
 against the SHA-256 of what the reference binary read -- the GPU `get` sees byte for byte the reference's input.
@@ -141,3 +144,45 @@ def test_detect_speed_10min_vs_reference(hour16, idx):
     speed_hits = [m for m in doc["matches"] if m["type"].endswith("-SPEED") and m["bits"] == PAYLOAD]
     assert n_real >= 10 and len(speed_hits) >= 10
     assert all(abs(m["speed"] - g["speed"]) < 1e-4 for m in speed_hits)
+
+
+# ---- tonal, quiet, clipped, one-sided stereo, mono and 3-channel inputs (tests/awm_testlib.py signals), watermarked by the reference
+MUSIC_CASES = ["music130", "tone170", "quiet130", "dc_clip130", "r_zero130", "r_m50_130", "r_same130", "r_neg130", "mono170", "ch3_170",
+               "music600"]
+
+
+@pytest.mark.parametrize("name", MUSIC_CASES)
+def test_music_cases_vs_reference(name):
+    """add against the oracle (RMS < 1e-5, at most 1 LSB apart on the 16 bit grid), then get on the reference's output: the whole
+    document, every sync position identical (none one fine step off), and the same document from the 16 bit entry point"""
+    g = G[name]
+    x = T.signal(g["signal"])
+    assert sha16(O.quantize_sndfile16(x)) == g["input_sha256"]
+    H.set_params()
+    y = H.add(x, PAYLOAD)
+    ref = O.embed(x, O.Key(), PAYLOAD, O.Params()).samples
+    assert T.rms(y - ref) < 1e-5, T.rms(y - ref)
+    y16, ref16 = O.quantize_sndfile16(y), O.quantize_sndfile16(ref)
+    assert np.abs(y16.astype(np.int32) - ref16).max() <= 1
+    assert sha16(ref16) == g["output_sha256"]
+    doc, trace = get_with_trace(O.int16_to_float(ref16))
+    n_real = compare_docs(doc, g["json"])
+    assert n_real >= 1 and any(m["bits"] == PAYLOAD for m in doc["matches"])
+    n_scores = sum(len(s["scores"]) for s in g["sync"])
+    assert compare_sync(trace, g["sync"]) == (n_scores, 0)
+    assert H.get_s16(ref16) == doc
+
+
+def test_music600_two_keys_vs_reference():
+    """the 10 min music-like input watermarked once with each of two named keys; get with both keys"""
+    g = G["music600_two_keys"]
+    ka = O.Key(bytes.fromhex(g["keys"]["alpha"]), "alpha")
+    kb = O.Key(bytes.fromhex(g["keys"]["beta"]), "beta")
+    x = T.signal(g["signal"])
+    y1 = O.int16_to_float(O.quantize_sndfile16(O.embed(x, ka, g["payload"], O.Params()).samples))
+    y16 = O.quantize_sndfile16(O.embed(y1, kb, g["payload2"], O.Params()).samples)
+    assert sha16(y16) == g["output_sha256"]
+    H.set_params()
+    doc = H.get(O.int16_to_float(y16), [ka.aes_key, kb.aes_key], ["alpha", "beta"])
+    assert compare_docs(doc, g["json"]) >= 2
+    assert {(m["key"], m["bits"]) for m in doc["matches"] if m["quality"] > 0.35} >= {("alpha", g["payload"]), ("beta", g["payload2"])}
