@@ -29,6 +29,7 @@ EXPORTS = [
     "awm_fft_r2c", "awm_fft_c2r", "awm_set_embed_tables", "awm_set_sync_tables", "awm_set_mix_tables",
     "awm_pcm_bind", "awm_pcm_prefetch", "awm_embed", "awm_sync_approx", "awm_sync_peaks", "awm_sync_refine", "awm_sync_refine_offsets", "awm_decode_blocks", "awm_viterbi",
     "awm_resample", "awm_pcm_push_resampled", "awm_pcm_pop", "awm_copy_to_host", "awm_is_device_pointer", "awm_speed_scan", "awm_embed_resampled", "awm_gather", "awm_pcm_bind_s16", "awm_pcm_prefetch_s16", "awm_pcm_device", "awm_embed_s16", "awm_embed_window", "awm_pcm_stage", "awm_pcm_stage_wait", "awm_dist_unique_id", "awm_dist_init", "awm_dist_world", "awm_dist_allgather",
+    "awm_pcm_bind_wav", "awm_pcm_prefetch_wav",
 ]
 
 _lib = None
@@ -60,6 +61,11 @@ def _ptr(x):
 
 class AwmError(RuntimeError):
     pass
+
+
+class WavFormat(ctypes.Structure):
+    """awm_wav_format: how WAV samples are stored (8 bit unsigned, 16/24/32 bit signed, 32/64 bit float; little endian)"""
+    _fields_ = [("bits", ctypes.c_int), ("is_float", ctypes.c_int)]
 
 
 class Context:
@@ -165,6 +171,40 @@ class Context:
                                        ctypes.c_size_t(pad_start), ctypes.c_size_t(pad_end)))
         if host or pad_start or pad_end:        # the asynchronous copy reads the caller's array; a device pointer is bound in place
             self.synchronize()
+
+    def pcm_bind_wav(self, data, bits: int, is_float: bool, n_frames: int, channels: int, pad_start: int = 0, pad_end: int = 0, offset: int = 0):
+        """bind stored WAV sample bytes (numpy uint8 / bytes from byte `offset` on, or a device pointer), decoded on the device"""
+        ptr = self._bytes_ptr(data, offset)
+        self._ck(self.lib.awm_pcm_bind_wav(self.h, ptr, WavFormat(bits, int(is_float)), ctypes.c_size_t(n_frames), ctypes.c_int(channels),
+                                           ctypes.c_size_t(pad_start), ctypes.c_size_t(pad_end)))
+        self.synchronize()
+
+    def pcm_prefetch_wav(self, data, bits: int, is_float: bool, n_frames: int, channels: int, head_frames: int = 0, offset: int = 0):
+        """start copying a span of stored WAV samples; its first head_frames frames come from the span prefetched before it and
+        `data` (from byte `offset` on) holds the rest.  Bind it with pcm_bind_wav (same data / offset, full n_frames)."""
+        ptr = self._bytes_ptr(data, offset)
+        self._ck(self.lib.awm_pcm_prefetch_wav(self.h, ptr, WavFormat(bits, int(is_float)), ctypes.c_size_t(n_frames), ctypes.c_int(channels),
+                                               ctypes.c_size_t(head_frames)))
+
+    def _bytes_ptr(self, data, offset):
+        if isinstance(data, (int, np.integer)):
+            return ctypes.c_void_p(int(data) + offset)
+        if not isinstance(data, np.ndarray):
+            data = np.frombuffer(data, np.uint8)
+        data = np.ascontiguousarray(data).view(np.uint8).reshape(-1)
+        self._keep_bytes = getattr(self, "_keep_bytes", [])[-3:] + [data]     # the copies read the array asynchronously
+        return ctypes.c_void_p(data.ctypes.data + offset)
+
+    def pcm_device(self):
+        """(device pointer, frames, channels) of the bound PCM (float32, padding included)"""
+        self.lib.awm_pcm_device.restype = ctypes.c_void_p
+        n, ch = ctypes.c_size_t(), ctypes.c_int()
+        p = self.lib.awm_pcm_device(self.h, ctypes.byref(n), ctypes.byref(ch))
+        return int(p or 0), n.value, ch.value
+
+    def copy_to_host(self, dst: np.ndarray, src_ptr: int):
+        self._ck(self.lib.awm_copy_to_host(self.h, _ptr(dst), ctypes.c_void_p(src_ptr), ctypes.c_size_t(dst.nbytes)))
+        return dst
 
     # ---- embed
     def embed(self, pcm_in, pcm_out=None, n_frames=None, channels=None, first_frame_number=0, frames_pad_start=250,

@@ -5,6 +5,7 @@
 // fallback: every entry point launches the sm_100a kernels of awm_kernels.cuh or fails.
 #include "awm_kernels.cuh"
 #include "awm_speed.cuh"
+#include "awm_wav_decode.cuh"
 #include "awm_refine_slide.cuh"
 #include "awm_approx_mags.cuh"
 #include <vector>
@@ -131,6 +132,9 @@ struct KeyTab
   int n_mix = 0, n_coded = 0, frames_per_bit = 0, fpb = 0;
 };
 
+/* sample layouts of the PCM entry points: the float pipeline's own samples (no conversion), or stored WAV samples (WavSampleType) */
+constexpr int kPcmFloat = -1;
+
 } // namespace
 
 struct awm_ctx
@@ -152,7 +156,9 @@ struct awm_ctx
   // bound PCM
   const float *pcm = nullptr; size_t pcm_frames = 0; int pcm_ch = 0;
   DevBuf pcm_own, pcm16_own;
-  struct Prefetch { DevBuf buf, buf16; bool s16 = false; const void *src = nullptr; size_t n_frames = 0; int ch = 0; cudaEvent_t done = nullptr; bool valid = false; };   // s16: buf16 holds the copy, it becomes float in buf when it is bound
+  /* one prefetched span.  type kPcmFloat: buf holds the copy; a WAV sample type: raw holds the stored bytes, they become float in buf
+   * when the span is bound, and stay in raw (the next span may take its head from there) until the slot is prefetched into again */
+  struct Prefetch { DevBuf buf, raw; int type = kPcmFloat; const void *src = nullptr; size_t n_frames = 0; int ch = 0; cudaEvent_t done = nullptr; bool valid = false, filled = false; };
   Prefetch pref[2];
   int pref_next = 0;
   /* awm_pcm_stage: a host stream on its way into `staged` piece by piece */
@@ -248,6 +254,59 @@ is_device_ptr (const void *p)
       return false;
     }
   return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+}
+
+int
+pcm_sample_bytes (int type)
+{
+  switch (type)
+    {
+    case WAV_U8:  return 1;
+    case WAV_S16: return 2;
+    case WAV_S24: return 3;
+    case WAV_F64: return 8;
+    default:      return 4;
+    }
+}
+
+/* awm_wav_format -> WavSampleType; -1 for a format no WAV input of `get` can have */
+int
+wav_sample_type (awm_wav_format f)
+{
+  if (f.is_float)
+    return f.bits == 32 ? WAV_F32 : f.bits == 64 ? WAV_F64 : -1;
+  switch (f.bits)
+    {
+    case 8:  return WAV_U8;
+    case 16: return WAV_S16;
+    case 24: return WAV_S24;
+    case 32: return WAV_S32;
+    default: return -1;
+    }
+}
+
+/* k_wav_to_f32 for a sample type known at run time: n samples at `in` (any byte address) -> out.  Profiled when it runs on the
+ * context stream (the profile events live there). */
+int
+wav_to_f32 (awm_ctx *ctx, int type, const void *in, float *out, long long n, cudaStream_t st)
+{
+  if (n <= 0)
+    return 0;
+  const unsigned grid = unsigned (((n + 3) / 4 + 255) / 256);
+  const unsigned char *b = static_cast<const unsigned char *> (in);
+  if (st == ctx->stream)
+    PROF (ctx);
+  switch (type)
+    {
+    case WAV_U8:  k_wav_to_f32<WAV_U8><<<grid, 256, 0, st>>> (b, out, n);  LAUNCH_CHECK ("k_wav_to_f32<u8>");  break;
+    case WAV_S16: k_wav_to_f32<WAV_S16><<<grid, 256, 0, st>>> (b, out, n); LAUNCH_CHECK ("k_wav_to_f32<s16>"); break;
+    case WAV_S24: k_wav_to_f32<WAV_S24><<<grid, 256, 0, st>>> (b, out, n); LAUNCH_CHECK ("k_wav_to_f32<s24>"); break;
+    case WAV_S32: k_wav_to_f32<WAV_S32><<<grid, 256, 0, st>>> (b, out, n); LAUNCH_CHECK ("k_wav_to_f32<s32>"); break;
+    case WAV_F32: k_wav_to_f32<WAV_F32><<<grid, 256, 0, st>>> (b, out, n); LAUNCH_CHECK ("k_wav_to_f32<f32>"); break;
+    case WAV_F64: k_wav_to_f32<WAV_F64><<<grid, 256, 0, st>>> (b, out, n); LAUNCH_CHECK ("k_wav_to_f32<f64>"); break;
+    default:      return fail (ctx, "wav_to_f32: unknown sample type %d", type);
+    }
+  return 0;
 }
 
 double
@@ -379,7 +438,7 @@ awm_destroy (awm_ctx *ctx)
   for (auto& pf : ctx->pref)
     {
       pf.buf.release();
-      pf.buf16.release();
+      pf.raw.release();
       if (pf.done)
         cudaEventDestroy (pf.done);
     }
@@ -681,37 +740,31 @@ awm_set_mix_tables (awm_ctx *ctx, int key_slot, const awm_mix_entry *entries, in
 
 namespace {
 
-/* awm_pcm_bind / awm_pcm_bind_s16 */
+/* awm_pcm_bind / awm_pcm_bind_s16 / awm_pcm_bind_wav: `type` is kPcmFloat or a WavSampleType */
 int
-pcm_bind_any (awm_ctx *ctx, const void *pcm_v, bool s16, size_t n_frames, int channels, size_t pad_start, size_t pad_end)
+pcm_bind_any (awm_ctx *ctx, const void *pcm_v, int type, size_t n_frames, int channels, size_t pad_start, size_t pad_end)
 {
   if (channels <= 0 || (!pcm_v && n_frames))
     return fail (ctx, "awm_pcm_bind: bad arguments");
   CK (cudaSetDevice (ctx->device));
   ctx->pushed = false;                           // a new bind replaces whatever awm_pcm_push_resampled saved
-  const float *pcm = s16 ? nullptr : static_cast<const float *> (pcm_v);
   const bool dev = pcm_v && is_device_ptr (pcm_v);
   awm_ctx::Prefetch *hit = nullptr;
   if (!dev && pad_start == 0 && pad_end == 0)
     for (auto& pf : ctx->pref)
-      if (pf.valid && pf.src == pcm_v && pf.n_frames == n_frames && pf.ch == channels && pf.s16 == s16)
+      if (pf.valid && pf.src == pcm_v && pf.n_frames == n_frames && pf.ch == channels && pf.type == type)
         hit = &pf;
   if (hit)
     {
       CK (cudaStreamWaitEvent (ctx->stream, hit->done, 0));   // the prefetched copy becomes the bound PCM
-      if (hit->s16)
-        {
-          const long long n_val = (long long) (n_frames * channels);
-          PROF (ctx);
-          k_s16_to_f32<<<unsigned (((n_val + 1) / 2 + 255) / 256), 256, 0, ctx->stream>>> (hit->buf16.as<int16_t>(), hit->buf.as<float>(), n_val);
-          LAUNCH_CHECK ("k_s16_to_f32");
-        }
+      if (hit->type != kPcmFloat && wav_to_f32 (ctx, hit->type, hit->raw.p, hit->buf.as<float>(), (long long) (n_frames * channels), ctx->stream))
+        return 1;
       ctx->pcm = hit->buf.as<float>();
       hit->valid = false;
     }
-  else if (dev && !s16 && pad_start == 0 && pad_end == 0)
+  else if (dev && type == kPcmFloat && pad_start == 0 && pad_end == 0)
     {
-      ctx->pcm = pcm;
+      ctx->pcm = static_cast<const float *> (pcm_v);
     }
   else
     {
@@ -720,22 +773,21 @@ pcm_bind_any (awm_ctx *ctx, const void *pcm_v, bool s16, size_t n_frames, int ch
       float *d = ctx->pcm_own.as<float>();
       if (pad_start)
         CK (cudaMemsetAsync (d, 0, pad_start * channels * sizeof (float), ctx->stream));
-      if (n_frames && !s16)
-        CK (cudaMemcpyAsync (d + pad_start * channels, pcm, n_frames * channels * sizeof (float),
+      if (n_frames && type == kPcmFloat)
+        CK (cudaMemcpyAsync (d + pad_start * channels, pcm_v, n_frames * channels * sizeof (float),
                              dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, ctx->stream));
-      if (n_frames && s16)
+      if (n_frames && type != kPcmFloat)
         {
-          const int16_t *src16 = static_cast<const int16_t *> (pcm_v);
-          const long long n_val = (long long) (n_frames * channels);
-          if (!dev)
+          const void *src = pcm_v;
+          const size_t n_val = n_frames * channels;
+          if (!dev)                                 // the stored bytes cross PCIe, they become float on the device
             {
-              CK (ctx->pcm16_own.reserve (n_val * sizeof (int16_t)));
-              CK (cudaMemcpyAsync (ctx->pcm16_own.p, src16, n_val * sizeof (int16_t), cudaMemcpyHostToDevice, ctx->stream));
-              src16 = ctx->pcm16_own.as<int16_t>();
+              CK (ctx->pcm16_own.reserve (n_val * pcm_sample_bytes (type)));
+              CK (cudaMemcpyAsync (ctx->pcm16_own.p, pcm_v, n_val * pcm_sample_bytes (type), cudaMemcpyHostToDevice, ctx->stream));
+              src = ctx->pcm16_own.p;
             }
-          PROF (ctx);
-          k_s16_to_f32<<<unsigned (((n_val + 1) / 2 + 255) / 256), 256, 0, ctx->stream>>> (src16, d + pad_start * channels, n_val);
-          LAUNCH_CHECK ("k_s16_to_f32");
+          if (wav_to_f32 (ctx, type, src, d + pad_start * channels, (long long) n_val, ctx->stream))
+            return 1;
         }
       if (pad_end)
         CK (cudaMemsetAsync (d + (pad_start + n_frames) * channels, 0, pad_end * channels * sizeof (float), ctx->stream));
@@ -746,20 +798,34 @@ pcm_bind_any (awm_ctx *ctx, const void *pcm_v, bool s16, size_t n_frames, int ch
   return 0;
 }
 
+/* awm_pcm_prefetch / awm_pcm_prefetch_s16 / awm_pcm_prefetch_wav.  head_frames = kFindHead: the head is found by pointer arithmetic
+ * (a span that starts inside the unbound span prefetched just before it, in the same host buffer); otherwise the first head_frames
+ * frames of this span are the last head_frames frames of the span prefetched just before it, and `pcm` holds the rest. */
+constexpr size_t kFindHead = ~size_t (0);
+
 int
-pcm_prefetch_any (awm_ctx *ctx, const void *pcm, bool s16, size_t n_frames, int channels)
+pcm_prefetch_any (awm_ctx *ctx, const void *pcm, int type, size_t n_frames, int channels, size_t head_frames)
 {
-  if (!pcm || !n_frames || channels <= 0)
+  const bool explicit_head = head_frames != kFindHead;
+  if (!n_frames || channels <= 0 || (explicit_head && head_frames > n_frames) || (!pcm && (!explicit_head || head_frames < n_frames)))
     return fail (ctx, "awm_pcm_prefetch: bad arguments");
   CK (cudaSetDevice (ctx->device));
-  if (is_device_ptr (pcm))
-    return 0;                                     // nothing to do: device memory is bound in place
+  if (pcm && is_device_ptr (pcm))
+    {
+      if (explicit_head && head_frames)
+        return fail (ctx, "awm_pcm_prefetch: a span with a head from the previous span must be in host memory");
+      return 0;                                   // nothing to do: device memory is bound in place
+    }
   if (!ctx->s_in)
     {
       CK (cudaStreamCreateWithFlags (&ctx->s_in, cudaStreamNonBlocking));
       CK (cudaStreamCreateWithFlags (&ctx->s_out, cudaStreamNonBlocking));
     }
   awm_ctx::Prefetch& pf = ctx->pref[ctx->pref_next];
+  awm_ctx::Prefetch& prev = ctx->pref[ctx->pref_next ^ 1];
+  const size_t esz = size_t (type == kPcmFloat ? sizeof (float) : pcm_sample_bytes (type)) * size_t (channels);   // bytes per frame
+  if (explicit_head && head_frames && !(prev.filled && prev.type == type && prev.ch == channels && prev.n_frames >= head_frames))
+    return fail (ctx, "awm_pcm_prefetch: the previous span (%zu frames) cannot supply a head of %zu frames in this format", prev.n_frames, head_frames);
   /* the slot's previous contents may still be the bound PCM of kernels in flight: order the copy behind them */
   cudaEvent_t busy;
   CK (cudaEventCreateWithFlags (&busy, cudaEventDisableTiming));
@@ -770,51 +836,73 @@ pcm_prefetch_any (awm_ctx *ctx, const void *pcm, bool s16, size_t n_frames, int 
     ctx->pcm_ch = 0;                              // the bound PCM is about to be overwritten: force a new bind
   const size_t n_val = n_frames * channels;
   CK (pf.buf.reserve (n_val * sizeof (float)));
+  if (type != kPcmFloat)
+    CK (pf.raw.reserve (n_frames * esz));
   if (!pf.done)
     CK (cudaEventCreateWithFlags (&pf.done, cudaEventDisableTiming));
-  /* Consecutive chunks of `get` overlap (WavChunkLoader: 134 s of 30 min).  When this span starts inside the span that was prefetched
-   * just before it and is still waiting to be bound, its head is already on the device: it is copied from there (device to device,
-   * ordered behind that upload on the same stream) and only the rest crosses PCIe -- 7 % fewer bytes for a 1 h stream. */
-  size_t head = 0;                              // frames taken from the previous prefetch
-  if (s16)
-    CK (pf.buf16.reserve (n_val * sizeof (int16_t)));
-  {
-    awm_ctx::Prefetch& prev = ctx->pref[ctx->pref_next ^ 1];
-    const size_t esz = (s16 ? sizeof (int16_t) : sizeof (float)) * size_t (channels);
-    const char *b0 = static_cast<const char *> (prev.src), *p0 = static_cast<const char *> (pcm);
-    if (prev.valid && prev.s16 == s16 && prev.ch == channels && b0 && p0 > b0 && p0 < b0 + prev.n_frames * esz && size_t (p0 - b0) % esz == 0)
-      {
-        const size_t first = size_t (p0 - b0) / esz;
-        head = std::min (prev.n_frames - first, n_frames);
-        if (s16)            // 16 bit audio stays 16 bit until it is bound (see below)
-          CK (cudaMemcpyAsync (pf.buf16.p, prev.buf16.as<int16_t>() + first * channels, head * channels * sizeof (int16_t), cudaMemcpyDeviceToDevice, ctx->s_in));
-        else
-          CK (cudaMemcpyAsync (pf.buf.p, prev.buf.as<float>() + first * channels, head * channels * sizeof (float), cudaMemcpyDeviceToDevice, ctx->s_in));
-      }
-  }
-  /* the copy stream carries copies only: the int -> float conversion of 16 bit audio runs on the context stream when the chunk is
-   * bound (pcm_bind_any), so the copy of the next chunk starts the moment this one has arrived */
-  const size_t rest = (n_frames - head) * channels, head_val = head * channels;
-  if (rest && s16)
-    CK (cudaMemcpyAsync (pf.buf16.as<int16_t>() + head_val, static_cast<const int16_t *> (pcm) + head_val, rest * sizeof (int16_t), cudaMemcpyHostToDevice, ctx->s_in));
-  else if (rest)
-    CK (cudaMemcpyAsync (pf.buf.as<float>() + head_val, static_cast<const float *> (pcm) + head_val, rest * sizeof (float), cudaMemcpyHostToDevice, ctx->s_in));
+  /* WAV samples stay in their stored format on the copy stream: they become float on the context stream when the span is bound
+   * (pcm_bind_any), so the copy of the next span starts the moment this one has arrived */
+  unsigned char *dst = static_cast<unsigned char *> (type == kPcmFloat ? pf.buf.p : pf.raw.p);
+  const unsigned char *prev_bytes = static_cast<const unsigned char *> (prev.type == kPcmFloat ? prev.buf.p : prev.raw.p);
+  /* Consecutive chunks of `get` overlap (WavChunkLoader: 134 s of 30 min).  The head of this span that is already on the device is
+   * copied from there (device to device, ordered behind that upload on the same stream) and only the rest crosses PCIe -- 7 % fewer
+   * bytes for a 1 h stream. */
+  size_t head = 0;
+  if (explicit_head)
+    {
+      head = head_frames;
+      if (head)
+        CK (cudaMemcpyAsync (dst, prev_bytes + (prev.n_frames - head) * esz, head * esz, cudaMemcpyDeviceToDevice, ctx->s_in));
+    }
+  else
+    {
+      const char *b0 = static_cast<const char *> (prev.src), *p0 = static_cast<const char *> (pcm);
+      if (prev.valid && prev.type == type && prev.ch == channels && b0 && p0 > b0 && p0 < b0 + prev.n_frames * esz && size_t (p0 - b0) % esz == 0)
+        {
+          const size_t first = size_t (p0 - b0) / esz;
+          head = std::min (prev.n_frames - first, n_frames);
+          CK (cudaMemcpyAsync (dst, prev_bytes + first * esz, head * esz, cudaMemcpyDeviceToDevice, ctx->s_in));
+        }
+    }
+  /* explicit head: `pcm` points at the frames after the head; found head: `pcm` is the whole span */
+  const unsigned char *host = static_cast<const unsigned char *> (pcm) + (explicit_head ? 0 : head * esz);
+  if (n_frames > head)
+    CK (cudaMemcpyAsync (dst + head * esz, host, (n_frames - head) * esz, cudaMemcpyHostToDevice, ctx->s_in));
   CK (cudaEventRecord (pf.done, ctx->s_in));
   pf.src = pcm;
   pf.n_frames = n_frames;
   pf.ch = channels;
-  pf.s16 = s16;
+  pf.type = type;
   pf.valid = true;
+  pf.filled = true;
   ctx->pref_next ^= 1;
   return 0;
 }
 
 } // namespace
 
-int awm_pcm_bind (awm_ctx *ctx, const float *pcm, size_t n_frames, int channels, size_t pad_start, size_t pad_end) { return pcm_bind_any (ctx, pcm, false, n_frames, channels, pad_start, pad_end); }
-int awm_pcm_bind_s16 (awm_ctx *ctx, const int16_t *pcm, size_t n_frames, int channels, size_t pad_start, size_t pad_end) { return pcm_bind_any (ctx, pcm, true, n_frames, channels, pad_start, pad_end); }
-int awm_pcm_prefetch (awm_ctx *ctx, const float *pcm, size_t n_frames, int channels) { return pcm_prefetch_any (ctx, pcm, false, n_frames, channels); }
-int awm_pcm_prefetch_s16 (awm_ctx *ctx, const int16_t *pcm, size_t n_frames, int channels) { return pcm_prefetch_any (ctx, pcm, true, n_frames, channels); }
+int awm_pcm_bind (awm_ctx *ctx, const float *pcm, size_t n_frames, int channels, size_t pad_start, size_t pad_end) { return pcm_bind_any (ctx, pcm, kPcmFloat, n_frames, channels, pad_start, pad_end); }
+int awm_pcm_bind_s16 (awm_ctx *ctx, const int16_t *pcm, size_t n_frames, int channels, size_t pad_start, size_t pad_end) { return pcm_bind_any (ctx, pcm, WAV_S16, n_frames, channels, pad_start, pad_end); }
+int awm_pcm_prefetch (awm_ctx *ctx, const float *pcm, size_t n_frames, int channels) { return pcm_prefetch_any (ctx, pcm, kPcmFloat, n_frames, channels, kFindHead); }
+int awm_pcm_prefetch_s16 (awm_ctx *ctx, const int16_t *pcm, size_t n_frames, int channels) { return pcm_prefetch_any (ctx, pcm, WAV_S16, n_frames, channels, kFindHead); }
+
+int
+awm_pcm_bind_wav (awm_ctx *ctx, const void *bytes, awm_wav_format format, size_t n_frames, int channels, size_t pad_start, size_t pad_end)
+{
+  const int type = wav_sample_type (format);
+  if (type < 0)
+    return fail (ctx, "awm_pcm_bind_wav: unsupported sample format (%d bit, %s)", format.bits, format.is_float ? "float" : "integer");
+  return pcm_bind_any (ctx, bytes, type, n_frames, channels, pad_start, pad_end);
+}
+
+int
+awm_pcm_prefetch_wav (awm_ctx *ctx, const void *bytes, awm_wav_format format, size_t n_frames, int channels, size_t head_frames)
+{
+  const int type = wav_sample_type (format);
+  if (type < 0)
+    return fail (ctx, "awm_pcm_prefetch_wav: unsupported sample format (%d bit, %s)", format.bits, format.is_float ? "float" : "integer");
+  return pcm_prefetch_any (ctx, bytes, type, n_frames, channels, head_frames);
+}
 
 /* awm_pcm_stage / awm_pcm_stage_wait: see include/awm_b200.h */
 int
@@ -840,7 +928,7 @@ awm_pcm_stage (awm_ctx *ctx, const void *pcm, int is_s16, size_t n_frames, int c
   CK (ctx->staged.reserve (n_val * sizeof (float)));
   if (is_s16)
     CK (ctx->staged16.reserve (n_val * sizeof (int16_t)));
-  piece_frames = (piece_frames + 1) & ~size_t (1);               // even: the conversion kernel stores float pairs
+  piece_frames = (piece_frames + 1) & ~size_t (1);               // even: pieces start on 4-byte boundaries of the 16 bit copy
   const size_t n_pieces = (n_frames + piece_frames - 1) / piece_frames;
   while (ctx->stage_done.size() < n_pieces)
     {
@@ -880,10 +968,8 @@ awm_pcm_stage_wait (awm_ctx *ctx, size_t n_frames)
     {
       const size_t f0 = ctx->stage_converted * ctx->stage_piece, f1 = std::min (f0 + ctx->stage_piece, ctx->stage_frames);
       const size_t v0 = f0 * ctx->stage_ch;
-      const long long nv = (long long) ((f1 - f0) * ctx->stage_ch);
-      PROF (ctx);
-      k_s16_to_f32<<<unsigned (((nv + 1) / 2 + 255) / 256), 256, 0, ctx->stream>>> (ctx->staged16.as<int16_t>() + v0, ctx->staged.as<float>() + v0, nv);
-      LAUNCH_CHECK ("k_s16_to_f32");
+      if (wav_to_f32 (ctx, WAV_S16, ctx->staged16.as<int16_t>() + v0, ctx->staged.as<float>() + v0, (long long) ((f1 - f0) * ctx->stage_ch), ctx->stream))
+        return 1;
     }
   return 0;
 }
@@ -957,11 +1043,7 @@ embed_any (awm_ctx *ctx, const void *in_v, void *out_v, bool s16, size_t n_frame
     {
       if (v1 <= v0)
         return 0;
-      if (st == ctx->stream)          /* the profile events live on the context stream */
-        PROF (ctx);
-      k_s16_to_f32<<<unsigned (((v1 - v0 + 1) / 2 + 255) / 256), 256, 0, st>>> (d_in16 + v0, ctx->emb_in.as<float>() + v0, v1 - v0);
-      LAUNCH_CHECK ("k_s16_to_f32");
-      return 0;
+      return wav_to_f32 (ctx, WAV_S16, d_in16 + v0, ctx->emb_in.as<float>() + v0, v1 - v0, st);
     };
   auto to_s16 = [&] (long long v0, long long v1, cudaStream_t st) -> int
     {

@@ -9,6 +9,7 @@
 
 #include <algorithm>
 #include <math.h>
+#include <memory>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -299,6 +300,70 @@ awmh_get_s16 (const unsigned char *keys16, const char *const *names, int n_keys,
   if (rc)
     return rc;
   return result_json (result_set, mark_rate_frames, json_out, json_cap, n_patterns);
+}
+
+/* `get` on the stored sample bytes of a WAV file held in memory (n_bytes / (bits / 8 * n_channels) frames; 8 bit is unsigned as in
+ * WAV): at 44.1 kHz the streamed loader of the CLI runs over the buffer (get_watermark_stream; two page-locked chunk buffers, decoded
+ * on the device), piece_frames frames per read of the buffer (0: a chunk per read); other rates are converted on the host and
+ * resampled as a whole, as the CLI does.  Writes the --json document into json_out. */
+int
+awmh_get_wav (const unsigned char *keys16, const char *const *names, int n_keys, const unsigned char *data, size_t n_bytes, int n_channels,
+              int bits, int is_float, int sample_rate, size_t piece_frames, char *json_out, size_t json_cap, int *n_patterns)
+{
+  if (n_channels <= 0 || (bits != 8 && bits != 16 && bits != 24 && bits != 32 && bits != 64))
+    return 1;
+  std::vector<Key> key_list;
+  for (int k = 0; k < n_keys; k++)
+    key_list.push_back (make_key (keys16 + 16 * k, names ? names[k] : ""));
+  const size_t frame_bytes = size_t (bits / 8) * n_channels, n_frames = n_bytes / frame_bytes;
+  ResultSet result_set;
+  size_t mark_rate_frames = n_frames;
+  if (sample_rate == Params::mark_sample_rate)
+    {
+      size_t pos = 0;
+      auto source = [&] (unsigned char *dst, size_t count, size_t *n_read)
+        {
+          *n_read = std::min (count, n_frames - pos);
+          memcpy (dst, data + pos * frame_bytes, *n_read * frame_bytes);
+          pos += *n_read;
+          return Error (Error::Code::NONE);
+        };
+      Error read_err;
+      const int rc = get_watermark_stream (key_list, source, awm_wav_format { bits, is_float ? 1 : 0 }, n_channels, n_frames, piece_frames, result_set,
+                                           false, &mark_rate_frames, read_err);
+      if (rc)
+        return rc;
+    }
+  else
+    {
+      RawFormat format (n_channels, sample_rate, bits);
+      format.set_encoding (is_float ? Encoding::FLOAT : bits == 8 ? Encoding::UNSIGNED : Encoding::SIGNED);
+      Error err;
+      std::unique_ptr<RawConverter> conv (RawConverter::create (format, err));
+      if (err)
+        return 1;
+      std::vector<float> samples (n_frames * n_channels);
+      conv->from_raw (data, samples.data(), samples.size());
+      const int rc = get_watermark_buffer (key_list, samples.data(), n_frames, n_channels, sample_rate, result_set, false, &mark_rate_frames);
+      if (rc)
+        return rc;
+    }
+  return result_json (result_set, mark_rate_frames, json_out, json_cap, n_patterns);
+}
+
+/* test aid (CPU): RawConverter::from_raw of n_samples stored WAV samples (8 bit unsigned, 16/24/32 bit signed, 32/64 bit float,
+ * little endian), the host conversion the device decode (awm_pcm_bind_wav) must equal bit for bit */
+int
+awmh_wav_decode_host (const unsigned char *bytes, size_t n_samples, int bits, int is_float, float *out)
+{
+  RawFormat format (1, Params::mark_sample_rate, bits);
+  format.set_encoding (is_float ? Encoding::FLOAT : bits == 8 ? Encoding::UNSIGNED : Encoding::SIGNED);
+  Error err;
+  std::unique_ptr<RawConverter> conv (RawConverter::create (format, err));
+  if (err)
+    return 1;
+  conv->from_raw (bytes, out, n_samples);
+  return 0;
 }
 
 /* get_watermark on a buffer (host pointer; a device pointer is accepted for inputs longer than 3.1 blocks,

@@ -413,6 +413,26 @@ WavInputStream::read_frames (vector<float>& samples, size_t count)
   return err;
 }
 
+Error
+WavInputStream::read_raw_frames (unsigned char *bytes, size_t count, size_t *n_read, RawFormat *format)
+{
+  if (format)
+    *format = m_format;
+  *n_read = 0;
+  if (m_frames_left != N_FRAMES_UNKNOWN)
+    count = std::min (count, m_frames_left);
+  if (count == 0)
+    return Error::Code::NONE;
+  const size_t frame_bytes = size_t (m_format.bit_depth() / 8) * m_format.n_channels();
+  const size_t got = fread (bytes, frame_bytes, count, m_file);      /* whole frames only, as read_frames */
+  if (ferror (m_file))
+    return Error ("error reading sample data");
+  if (m_frames_left != N_FRAMES_UNKNOWN)
+    m_frames_left -= got;
+  *n_read = got;
+  return Error::Code::NONE;
+}
+
 /* ---------------------------------------------------------------- WAV output */
 
 WavOutputStream::~WavOutputStream()

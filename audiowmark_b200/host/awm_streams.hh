@@ -145,6 +145,11 @@ public:
   ~WavInputStream();
   Error    open (const std::string& filename, bool pipe_mode);
   Error    read_frames (std::vector<float>& samples, size_t count) override;
+  /* the undecoded sample bytes of up to `count` frames (what read_frames would convert) into bytes[0 .. count * frame size);
+   * *n_read = frames delivered, 0 at EOF.  *format (if given) = how the bytes are stored: bit depth, encoding (8 bit is UNSIGNED,
+   * float WAVs FLOAT, everything else SIGNED), little endian, channels, sample rate. */
+  Error    read_raw_frames (unsigned char *bytes, size_t count, size_t *n_read, RawFormat *format = nullptr);
+  const RawFormat& raw_format() const   { return m_format; }
   int      bit_depth() const override   { return m_format.bit_depth(); }
   int      sample_rate() const override { return m_format.sample_rate(); }
   int      n_channels() const override  { return m_format.n_channels(); }

@@ -39,6 +39,12 @@ int get_watermark_pcm (const std::vector<Key>& key_list, const float *samples, c
 int add_watermark_buffer_s16 (const Key& key, const int16_t *in, int16_t *out, size_t n_frames, int n_channels, int sample_rate,
                               const std::string& bits, AddStats *stats, uint64_t first_frame_number = 0);
 
+/* `get` on a stream of stored WAV samples at mark_sample_rate, read chunk by chunk (WavChunkLoader): source (dst, count, &n_read)
+ * delivers the bytes of up to count frames, n_read = 0 at the end.  The CLI reads a WavInputStream, awmh_get_wav a memory buffer. */
+int get_watermark_stream (const std::vector<Key>& key_list, const std::function<Error (unsigned char *, size_t, size_t *)>& source,
+                          awm_wav_format format, int n_channels, size_t n_frames_hint, size_t piece_frames, ResultSet& result_set,
+                          bool print_speed_results, size_t *n_frames_out, Error& read_error);
+
 /* chunk-level pieces of get_watermark_buffer for sharded runs (one process per GPU): a rank decodes some of the
  * reference's chunks (WavChunkLoader geometry) and the chunk result sets are merged in chunk order afterwards */
 int get_watermark_chunk (const std::vector<Key>& key_list, const float *samples, size_t n_frames, int n_channels, int sample_rate,

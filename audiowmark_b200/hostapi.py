@@ -16,7 +16,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libawm_host.so")
 CLI_PATH = os.path.join(_HERE, "bin", "audiowmark")
 
 EXPORTS = ["awmh_set_params", "awmh_frames_per_block", "awmh_n_coded_bits", "awmh_random_u64", "awmh_gen_noise", "awmh_sync_table",
-           "awmh_mix_table", "awmh_frame_mod", "awmh_conv_encode", "awmh_add", "awmh_get", "awmh_get_chunk", "awmh_merge_chunks", "awmh_chunk_geometry", "awmh_ctx", "awmh_key_slot", "awmh_stage_select", "awmh_stage_final", "awmh_stage_jobs", "awmh_gpu_launches", "awmh_gpu_stream", "awmh_synchronize", "awmh_profile_enable", "awmh_profile_report", "awmh_shutdown", "awmh_set_speed_params", "awmh_detect_speed", "awmh_resample", "awmh_resample_stream_frames", "awmh_resample_stream_available", "awmh_resampled_add_plan", "awmh_set_short_payload", "awmh_add_s16", "awmh_get_s16", "awmh_short_encode", "awmh_short_decode", "awmh_sync_trace", "awmh_sync_trace_fetch", "awmh_dist_unique_id", "awmh_dist_init", "awmh_balanced_get", "awmh_bg_create", "awmh_bg_destroy", "awmh_bg_stage", "awmh_bg_plan", "awmh_bg_owner", "awmh_add_windowed"]
+           "awmh_mix_table", "awmh_frame_mod", "awmh_conv_encode", "awmh_add", "awmh_get", "awmh_get_chunk", "awmh_merge_chunks", "awmh_chunk_geometry", "awmh_ctx", "awmh_key_slot", "awmh_stage_select", "awmh_stage_final", "awmh_stage_jobs", "awmh_gpu_launches", "awmh_gpu_stream", "awmh_synchronize", "awmh_profile_enable", "awmh_profile_report", "awmh_shutdown", "awmh_set_speed_params", "awmh_detect_speed", "awmh_resample", "awmh_resample_stream_frames", "awmh_resample_stream_available", "awmh_resampled_add_plan", "awmh_set_short_payload", "awmh_add_s16", "awmh_get_s16", "awmh_short_encode", "awmh_short_decode", "awmh_sync_trace", "awmh_sync_trace_fetch", "awmh_dist_unique_id", "awmh_dist_init", "awmh_balanced_get", "awmh_bg_create", "awmh_bg_destroy", "awmh_bg_stage", "awmh_bg_plan", "awmh_bg_owner", "awmh_add_windowed", "awmh_get_wav", "awmh_wav_decode_host"]
 
 _lib = None
 
@@ -194,6 +194,42 @@ def get(pcm, keys=None, names=None, n_frames=None, channels=None, sample_rate=44
         raise RuntimeError("awmh_get failed (rc=%d); see stderr" % rc)
     text = buf.value.decode()
     return json.loads(text) if parse else text
+
+
+def get_wav_bytes(data, channels, bits, is_float=False, sample_rate=44100, keys=None, names=None, chunk_buffer=None, parse=True):
+    """`get` on the stored sample bytes of a WAV file (bytes or numpy; 8 bit unsigned, 16/24/32 bit signed, 32/64 bit float, little
+    endian) -> the --json document.  At 44.1 kHz this is the CLI's streamed loader over a memory buffer: chunks are read into two
+    page-locked buffers and decoded on the device.  chunk_buffer: frames handed out per read of the buffer, as a pipe delivers short
+    reads (None: a whole chunk per read); it does not change the result."""
+    keys = keys or [bytes(16)]
+    names = names or [""] * len(keys)
+    if not isinstance(data, np.ndarray):
+        data = np.frombuffer(data, np.uint8)
+    data = np.ascontiguousarray(data).view(np.uint8).reshape(-1)
+    kb = b"".join(_key(k) for k in keys)
+    name_arr = (ctypes.c_char_p * len(keys))(*[n.encode() for n in names])
+    cap = 1 << 22
+    buf = _outbuf("get", cap)
+    n_pat = ctypes.c_int()
+    rc = load().awmh_get_wav(kb, name_arr, ctypes.c_int(len(keys)), _ptr(data), ctypes.c_size_t(data.nbytes), ctypes.c_int(channels),
+                             ctypes.c_int(bits), ctypes.c_int(int(is_float)), ctypes.c_int(sample_rate), ctypes.c_size_t(chunk_buffer or 0),
+                             buf, ctypes.c_size_t(cap), ctypes.byref(n_pat))
+    if rc:
+        raise RuntimeError("awmh_get_wav failed (rc=%d); see stderr" % rc)
+    text = buf.value.decode()
+    return json.loads(text) if parse else text
+
+
+def wav_decode_host(data, bits, is_float=False) -> np.ndarray:
+    """test aid: the host's RawConverter::from_raw of stored WAV sample bytes -> float32 (one value per sample)"""
+    if not isinstance(data, np.ndarray):
+        data = np.frombuffer(data, np.uint8)
+    data = np.ascontiguousarray(data).view(np.uint8).reshape(-1)
+    n = data.nbytes // (bits // 8)
+    out = np.empty(n, np.float32)
+    if load().awmh_wav_decode_host(_ptr(data), ctypes.c_size_t(n), ctypes.c_int(bits), ctypes.c_int(int(is_float)), _ptr(out)):
+        raise ValueError("unsupported sample format: %d bit %s" % (bits, "float" if is_float else "integer"))
+    return out
 
 
 def sync_trace(on=True):
